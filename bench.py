@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W              # this engine, one rank per GPU
     python bench.py --impl reference --gpus N --steps K ...    # the reference's CPU path
     python bench.py --workload second_encoder6_fp16 ...        # another BASELINE config as headline
+    python bench.py --dump-outputs DIR ...                     # + the last timed step's outputs as DIR/*.npy
 
 Headline workload = BASELINE.json configs[1] (the configuration the metric is quoted on): one
 SubMConv3d 3x3x3 C = K = 64 fp16 over a ~100 k-voxel KITTI-shaped cloud per GPU.  A "step" is one
@@ -61,6 +62,7 @@ METRIC = "active-voxels/sec fwd+bwd SubMConv3d 3^3 C=64"
 NUM_CLOUDS = 4          # distinct clouds per rank, rotated so consecutive steps never share inputs
 L2_FLUSH_BYTES = 256 << 20
 CPU_THREAD_CAP = 16     # the small per-offset GEMMs get SLOWER with more BLAS threads (measured: 128 -> 3.2 s/step)
+DUMP_BYTES = 60 << 20   # --dump-outputs budget (below 64 MB with the .npy headers); larger outputs are row-sampled
 
 
 def metric_name(workload: str) -> str:
@@ -75,7 +77,9 @@ def metric_name(workload: str) -> str:
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps: of each of the three repetitions of the headline workload's timed region, and "
+                         "of --impl reference; the extra workloads time max(5, min(steps, 10))")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
@@ -99,7 +103,14 @@ def parse_args():
     ap.add_argument("--debug-bits", type=int, default=0,
                     help="spx_debug_configure bits for A/B runs (64 onesweep sort, 128 round-1 conv rulebook, "
                          "512 cooperative sort); recorded in config.debug_bits")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step of the headline workload returned "
+                         "(output coordinates and features, gradients, loss) as DIR/<name>.npy in float32, at most "
+                         "64 MB in all (a seeded row sample of every array beyond that); rank 0 only")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ============================================================================ CPU reference arm
@@ -214,7 +225,7 @@ def run_reference(args):
     if rank != 0:
         return
     wl = WORKLOADS[args.workload]
-    cb, value, steps, tot = cpu_arm(wl, args.cpu_sample, max(1, min(args.steps, 3)), max(args.steps, 1), 120.0)
+    cb, value, steps, tot = cpu_arm(wl, args.cpu_sample, args.steps, args.steps, 0.0)
     line = {
         "impl": "reference", "metric": metric_name(args.workload), "value": value, "unit": "voxels/s",
         "n_gpus": args.gpus, "steps": steps, "warmup": 1, "ms_per_step": 1e3 * tot / steps,
@@ -312,6 +323,7 @@ class Workload:
     ``e2e_body`` (public module API on freshly copied inputs)."""
     graphable = False
     inference = False
+    record_outputs = False                       # --dump-outputs: steps keep references to what they returned
 
     def __init__(self, name: str, ctx: Ctx):
         self.name, self.ctx, self.wl = name, ctx, WORKLOADS[name]
@@ -351,6 +363,11 @@ class Workload:
     def e2e_body(self, d_inds, d_feats): return self.e2e_from_input(self.make_input(d_inds, d_feats))
     def config(self) -> dict: return {}
     def region_kinds(self) -> Dict[str, tuple]: return {}
+
+    def outputs(self, c) -> dict:
+        """What the last step run or captured on cloud ``c`` returned to its caller, by name (recorded only
+        while ``record_outputs`` is set)."""
+        return c["outputs"]
 
 
 class LayerWorkload(Workload):
@@ -398,6 +415,8 @@ class LayerWorkload(Workload):
                                               masks, True, self.wl["subm"], **kw)
         din, dw = ops.implicit_gemm_backward(c["d_feats"], weight, c["dout"], pair_fwd, pair_bwd, mask_fwd, mask_bwd,
                                              sort_fwd, sort_bwd, mask_out, masks, mw, self.wl["subm"], **kw)
+        if self.record_outputs:
+            c["outputs"] = {"out_indices": out_inds, "out_features": out, "input_grad": din, "weight_grad": dw}
         return out, din, dw
 
     def device_step(self, c, timer=None, calls=1):
@@ -511,6 +530,9 @@ class EncoderWorkload(Workload):
                 acts.append(m(acts[-1]))
         loss = acts[-1].features.square().mean(dtype=torch.float32)
         loss.backward()
+        if self.record_outputs:
+            self.last_outputs = {"out_indices": acts[-1].indices, "out_features": acts[-1].features.detach(),
+                                 "loss": loss.detach(), "input_grad": acts[0].features.grad, "weight_grads": self.bucket.flat}
         if self.layer_stats is None:
             self.layer_stats = [(int(a.features.shape[0]), int(b.features.shape[0])) for a, b in zip(acts[:-1], acts[1:])]
             self.pairs = []
@@ -537,6 +559,9 @@ class EncoderWorkload(Workload):
 
     def grads(self):
         return self.bucket.flat
+
+    def outputs(self, c):
+        return self.last_outputs                 # eager steps only: the last forward_backward is the last step
 
     def config(self):
         return {"grid": self.wl["shape"], "batch_per_gpu": self.batch, "active_voxels_per_gpu": int(self.n_per_step),
@@ -578,19 +603,21 @@ class Int8Workload(Workload):
                                                            [1] * 3, [1] * 3, [0] * 3, True, False, is_train=False, **kw)
 
     def compute(self, c, res):
-        return self.conv(c["d_feats"], res, {})
+        return self.conv(c["d_feats"], res, {}, c)
 
     def run(self, d_inds, d_feats, c, kw):
         res = self.ctx.ops.get_indice_pairs_implicit_gemm(d_inds, 1, self.wl["shape"], self.algo, [3] * 3, [1] * 3,
                                                           [1] * 3, [1] * 3, [0] * 3, True, False, is_train=False, **kw)
-        return self.conv(d_feats, res, kw)
+        return self.conv(d_feats, res, kw, c)
 
-    def conv(self, d_feats, res, kw):
+    def conv(self, d_feats, res, kw, c=None):
         from spconv_b200.core import Activation
         out_inds, _, pair_fwd, _, mask_fwd, _, sort_fwd, _, masks = res
         out, _, _ = self.ctx.ops.implicit_gemm(d_feats, self.weight, pair_fwd, mask_fwd, sort_fwd, out_inds.shape[0], masks,
                                                False, True, bias=self.bias, act_type=Activation.ReLU, scale=self.scale,
                                                output_dtype=self.ctx.torch.int8, **kw)
+        if c is not None and self.record_outputs:
+            c["outputs"] = {"out_indices": out_inds, "out_features": out}
         return out
 
     def device_step(self, c, timer=None):
@@ -620,13 +647,15 @@ def make_workload(name, ctx) -> Workload:
 
 
 # ============================================================================ GPU arm: measurement
-def measure(w: Workload, ctx: Ctx, steps: int, warmup: int, headline: bool) -> dict:
+def measure(w: Workload, ctx: Ctx, steps: int, warmup: int, headline: bool, dump_dir: Optional[str] = None) -> dict:
     """Times one workload: value (device-resident), e2e (graph when possible + eager), per-region
     kernel times and the roofline of the dominant GEMM region.  Returns a dict of results reduced
-    over ranks (max time, sum voxels)."""
+    over ranks (max time, sum voxels).  ``dump_dir``: where rank 0 writes the outputs of the last timed
+    step of ``value`` (see write_outputs)."""
     torch, dist, ops = ctx.torch, ctx.dist, ctx.ops
     from spconv_b200.pytorch.core import CUDAKernelTimer
     w.setup()
+    w.record_outputs = dump_dir is not None and ctx.rank == 0
     world = ctx.world
     clouds = w.clouds
     train = not w.inference
@@ -654,6 +683,7 @@ def measure(w: Workload, ctx: Ctx, steps: int, warmup: int, headline: bool) -> d
     # overlaps the rulebook generation of this step (which does not depend on weights) and is
     # joined before the forward pass -- exactly where an optimizer update would consume it.
     graphs = None
+    graph_outs = pipe_outs = None                # per cloud: the output tensors of its captured graph
     use_graph = bool(ctx.args.graph) and w.graphable
     if use_graph:
         try:
@@ -674,6 +704,7 @@ def measure(w: Workload, ctx: Ctx, steps: int, warmup: int, headline: bool) -> d
                         w.device_step(c)
                 graphs.append(g)
             torch.cuda.synchronize()
+            graph_outs = [c.get("outputs") for c in clouds]
         except Exception as e:                       # capture is an optimisation, never a requirement
             print(f"[bench] CUDA-graph capture failed ({type(e).__name__}: {e}); running eagerly", file=sys.stderr)
             graphs, use_graph = None, False
@@ -705,6 +736,7 @@ def measure(w: Workload, ctx: Ctx, steps: int, warmup: int, headline: bool) -> d
                 g.replay()
             torch.cuda.synchronize()
             pipe = (rb_graphs, ge_graphs)
+            pipe_outs = [c.get("outputs") for c in clouds]
         except Exception as e:
             print(f"[bench] pipelined capture failed ({type(e).__name__}: {e}); serial graph replay", file=sys.stderr)
             pipe = None
@@ -878,6 +910,15 @@ def measure(w: Workload, ctx: Ctx, steps: int, warmup: int, headline: bool) -> d
             value_step(i)
     runs = [float(np.mean(ctx.timed_loop(value_step, steps))) for _ in range(3)]
     ms_value = sorted(runs)[1]
+    dumped = None
+    if w.record_outputs:
+        # the last timed step ran cloud j.  A graph replay rewrites the tensors captured with the graph that
+        # value_step replays (eager steps outside the timed loop record other tensors); an eager timed step
+        # recorded its own.  Host copy now: the legs below run the same clouds again.
+        j = (steps - 1) % NUM_CLOUDS
+        outs = pipe_outs[j] if pipe is not None else graph_outs[j] if use_graph else w.outputs(clouds[j])
+        dumped = {k: t.detach().cpu() for k, t in outs.items()}
+        w.record_outputs = False
     ms_serial = float(np.mean(ctx.timed_loop(serial_step, steps))) if pipe is not None else None
     ms_e2e = float(np.mean(ctx.timed_loop(e2e_step, steps)))
     clocks = sampler.stop() if (ctx.rank == 0 and headline) else {}
@@ -962,7 +1003,22 @@ def measure(w: Workload, ctx: Ctx, steps: int, warmup: int, headline: bool) -> d
                         if getattr(w, "hooked", False) else ("NCCL: one flat bucket after backward" if explicit_ar else "none"))
     ops.set_wgrad_hook(None)
     ops.set_peer_group(None)
+    if dumped is not None:
+        write_outputs(dump_dir, dumped)
     return res
+
+
+def write_outputs(path: str, outputs: dict) -> None:
+    """``path/<name>.npy`` in float32 (float64 stays float64).  When the arrays exceed DUMP_BYTES, every array
+    keeps the same fraction of its rows, chosen by a fixed seed (identical rows from run to run)."""
+    arrays = {name: (t if str(t.dtype) == "torch.float64" else t.float()).numpy() for name, t in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES and a.ndim > 0 and a.shape[0] > 1:
+            keep = max(1, a.shape[0] * DUMP_BYTES // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 def roofline_of(w: Workload, regions: Dict[str, float]) -> Optional[dict]:
@@ -1017,7 +1073,7 @@ def run_ours(args):
     ctx = Ctx(args)
     world, rank = ctx.world, ctx.rank
     extras = args.extras if args.extras >= 0 else int(args.workload == DEFAULT_WORKLOAD)
-    head = measure(make_workload(args.workload, ctx), ctx, args.steps, args.warmup, True)
+    head = measure(make_workload(args.workload, ctx), ctx, args.steps, args.warmup, True, args.dump_outputs)
     others = {}
     if extras:
         # at N > 1 only the encoder (BASELINE configs[2] is the multi-GPU config) rides along: every

@@ -1,22 +1,25 @@
-"""Regenerates tests/golden/*.  Run in the build container only (needs /root/reference).
+"""Regenerates tests/golden/*.  Needs the reference source tree (``SPCONV_REFERENCE_ROOT``, see
+oracle/make_ref.py); the tests themselves only read the files written here.
 
+* ``reference_cpu.json``  -- what the reference's own CPU code (oracle/_ref) returns on every input of
+  tests/test_oracle_ref.py and tests/test_pointops_gpu.py: rulebooks, gather / scatter-add, max-pool
+  forward / backward / global rearrange, voxel generator.  Arrays are SHA-256 digests
+  (``tests.util.digest``); per-offset pair counts are stored as numbers.
 * ``fixture_coords.npz``  -- voxel coordinates of the reference's own LiDAR fixture
   (test/data/test_spconv.pkl: 125 562 voxels, shape [80, 1600, 1600]); data, not source.
 * ``fixture_facts.json``  -- rulebook facts of that fixture computed with an implementation that
   shares nothing with oracle/ (sorted linear keys + np.searchsorted): per-offset SubM pair counts,
   pair / output counts of SparseConv3d(k3, s2, p1).  BASELINE.md section 2 quotes the same totals.
-* ``dense_conv_case.npz`` -- one seeded dense-equivalence case of test/test_conv.py:247-357
-  (inputs + torch.nn.functional.conv3d outputs / input-grad / weight-grad), so the GPU box can
-  check the kernels against torch's dense conv without regenerating anything.
 """
 import json
 import os
 import pickle
+import sys
 
 import numpy as np
-import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
 
 def linear(c, shape):
@@ -26,8 +29,87 @@ def linear(c, shape):
     return k
 
 
+def reference_records():
+    """Runs the reference's own CPU code (oracle/_ref) on the inputs of the reference-parity tests."""
+    from oracle import oracle as orc
+    from tests import test_oracle_ref as t
+    from tests import test_pointops_gpu as tp
+    from tests.util import digest
+    assert orc.have_ref(), "oracle/_ref is not built: the reference source tree is needed"
+    rec = {"rulebook": {}}
+    rb = rec["rulebook"]
+
+    def ref_rulebook(key, inds, *args):
+        rb[key] = t.rulebook_record(inds, t.rulebook(orc, inds, *args, impl="ref"))
+
+    for case in t.CASES:
+        shape, pts, ksize, stride, padding, dilation, subm, transpose = case
+        for seed in t.SEEDS:
+            ref_rulebook(f"{t.case_id(case)}/{seed}", t.rulebook_case_input(case, seed), len(pts), shape, ksize,
+                         stride, padding, dilation, subm, transpose)
+    inds = t.duplicates_input()
+    ref_rulebook("duplicates/subm", inds, 1, [16] * 3, [3] * 3, [1] * 3, [1] * 3, [1] * 3, True, False)
+    ref_rulebook("duplicates/conv", inds, 1, [16] * 3, [3] * 3, [2] * 3, [1] * 3, [1] * 3, False, False)
+    inds, shape = t.lidar_fixture_input()
+    ref_rulebook("lidar/subm", inds, 1, shape, [3] * 3, [1] * 3, [1] * 3, [1] * 3, True, False)
+    ref_rulebook("lidar/conv", inds, 1, shape, [3] * 3, [2] * 3, [1] * 3, [1] * 3, False, False)
+    inds = t.kitti_surface_input()
+    ref_rulebook("kitti_surface/subm", inds, 2, [41, 1600, 1408], [3] * 3, [1] * 3, [1] * 3, [1] * 3, True, False)
+    ref_rulebook("kitti_surface/conv", inds, 2, [41, 1600, 1408], [3] * 3, [2] * 3, [1] * 3, [1] * 3, False, False)
+
+    src, inds, dst = t.gather_input()
+    r = orc.ref_lib()
+    buf = np.empty((3000, 24), np.float32)
+    rec_g = {"inputs": [digest(src), digest(inds), digest(dst)]}
+    r.ref_gather_f32(orc._ptr(buf), orc._ptr(src), orc._ptr(inds), 3000, 24, 5000)
+    r.ref_scatter_add_f32(orc._ptr(dst), orc._ptr(buf), orc._ptr(inds), 3000, 24, 5000)
+    rec_g.update(gather=digest(buf), scatter_add=digest(dst))
+    rec["gather_scatter"] = rec_g
+
+    _, inds = t.random_cloud(np.random.default_rng(0), [8, 8, 8], [50], 1)
+    try:
+        orc.get_indice_pairs(inds, 1, [8] * 3, [2] * 3, [1] * 3, [0] * 3, [1] * 3, [0] * 3, True, impl="ref")
+    except RuntimeError as e:
+        rec["subm_even_ksize_error"] = str(e)
+    assert "subm_even_ksize_error" in rec, "the reference accepted an even SubM kernel size"
+
+    rng, feats, inds = t.pooling_input()
+    ref_rulebook("pooling", inds, 2, [18, 20, 22], [3] * 3, [2] * 3, [1] * 3, [1] * 3, False, False)
+    o, pairs, num = t.rulebook(orc, inds, 2, [18, 20, 22], [3] * 3, [2] * 3, [1] * 3, [1] * 3, False, False,
+                               impl="ref")
+    fwd = orc.indice_maxpool(feats, pairs, num, o.shape[0])                      # the reference's loop
+    tabs = orc.implicit_gemm_tables(pairs, num, inds.shape[0], o.shape[0], False)
+    dense = orc.maxpool_implicit_gemm(feats, tabs["pair_fwd"], -3e38)
+    g = rng.standard_normal(fwd.shape).astype(np.float32)
+    bwd = orc.indice_maxpool_backward(feats, dense, g, pairs, num)               # the reference's loop
+    oi, cnt = orc.global_pool_rearrange(inds, 2)
+    rec["pooling"] = {"forward": digest(fwd), "grad_inputs": digest(g), "backward": digest(bwd),
+                      "rearrange": digest(oi), "rearrange_counts": digest(cnt)}
+
+    pts = t.point2voxel_input()
+    p2v = {"inputs": digest(pts)}
+    for max_voxels, max_points in t.P2V_LIMITS:
+        p2v[f"{max_voxels}x{max_points}"] = [digest(a) for a in orc.point2voxel_ref(pts, t.P2V_VS, t.P2V_CR,
+                                                                                      max_voxels, max_points)]
+    _, grid, stride, _ = orc.point2voxel_meta(t.P2V_VS, t.P2V_CR)
+    p2v["meta"] = {"grid": grid.tolist(), "stride": stride.tolist()}
+    rec["point2voxel"] = p2v
+    rec["point2voxel_gpu_cases"] = {}
+    for n, max_voxels, max_points in tp.P2V_CASES:
+        pts = tp._points(n, n)
+        out = orc.point2voxel_ref(pts, tp.VS, tp.CR, max_voxels, max_points)
+        rec["point2voxel_gpu_cases"][f"{n}/{max_voxels}x{max_points}"] = {
+            "inputs": digest(pts), "outputs": [digest(a) for a in out]}
+    return rec
+
+
 def main():
-    voxels, coors, shape = pickle.load(open("/root/reference/test/data/test_spconv.pkl", "rb"))
+    from oracle import make_ref
+    rec = reference_records()
+    with open(os.path.join(HERE, "reference_cpu.json"), "w") as f:
+        json.dump(rec, f, indent=1)
+        f.write("\n")
+    voxels, coors, shape = pickle.load(open(os.path.join(make_ref.REF_ROOT, "test", "data", "test_spconv.pkl"), "rb"))
     coors = np.ascontiguousarray(coors.astype(np.int32))
     np.savez_compressed(os.path.join(HERE, "fixture_coords.npz"), coors=coors,
                         shape=np.array(shape, np.int32))
@@ -66,45 +148,6 @@ def main():
              "conv_k3s2p1_out_shape": oshape}
     json.dump(facts, open(os.path.join(HERE, "fixture_facts.json"), "w"), indent=1)
     print(facts["subm_k3_pairs_total"], pairs, len(outs))
-
-    # dense-equivalence golden (test/test_conv.py:247-357 with its seeds and a small grid)
-    np.random.seed(484)
-    torch.manual_seed(48848)
-    shape3, bs, npts, C, K = [19, 18, 17], 2, 1500, 16, 16
-    total = int(np.prod(shape3))
-    inds = []
-    for b in range(bs):
-        flat = np.random.permutation(total)[:npts]
-        cc = np.stack(np.unravel_index(flat, shape3), -1).astype(np.int32)
-        inds.append(np.concatenate([np.full((npts, 1), b, np.int32), cc], 1))
-    inds = np.concatenate(inds, 0)
-    feats = np.random.uniform(-1, 1, size=(inds.shape[0], C)).astype(np.float32)
-    import sys
-    sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
-    from oracle import oracle as orc
-    out = {}
-    for tag, (k, s, p, d) in {"k3s2p1d1": (3, 2, 1, 1), "k3s1p1d1": (3, 1, 1, 1),
-                              "k2s2p0d1": (2, 2, 0, 1)}.items():
-        w = np.random.uniform(-1, 1, size=(K, k, k, k, C)).astype(np.float32)
-        dense = torch.zeros((bs, C, *shape3))
-        dense[inds[:, 0], :, inds[:, 1], inds[:, 2], inds[:, 3]] = torch.from_numpy(feats)
-        dense.requires_grad_(True)
-        wt = torch.from_numpy(w).permute(0, 4, 1, 2, 3).contiguous().requires_grad_(True)
-        y = torch.nn.functional.conv3d(dense, wt, stride=s, padding=p, dilation=d)
-        dy = torch.from_numpy(np.random.uniform(-0.2, 0.2, size=tuple(y.shape)).astype(np.float32))
-        # the sparse op only defines gradients through its ACTIVE outputs: mask dy to them
-        oi, _, _ = orc.get_indice_pairs(inds, bs, shape3, [k] * 3, [s] * 3, [p] * 3, [d] * 3, [0] * 3, False)
-        act = torch.zeros_like(y)
-        act[oi[:, 0], :, oi[:, 1], oi[:, 2], oi[:, 3]] = 1
-        assert float((y.detach() * (1 - act)).abs().max()) == 0.0      # inactive outputs are exactly 0
-        y.backward(dy * act)
-        out[f"{tag}_w"] = w
-        out[f"{tag}_y"] = y.detach().numpy()
-        out[f"{tag}_dy"] = dy.numpy()
-        out[f"{tag}_dw"] = wt.grad.permute(0, 2, 3, 4, 1).contiguous().numpy()      # back to KRSC
-        out[f"{tag}_dx"] = dense.grad[inds[:, 0], :, inds[:, 1], inds[:, 2], inds[:, 3]].numpy()
-    np.savez_compressed(os.path.join(HERE, "dense_conv_case.npz"), inds=inds, feats=feats,
-                        shape=np.array(shape3), **out)
 
 
 if __name__ == "__main__":

@@ -1,16 +1,13 @@
 """Module-level GPU tests: the reference's dense-equivalence test (test/test_conv.py:247-357)
-run through SparseConv3d / SubMConv3d with autograd, against the committed torch golden vectors
-and against live torch conv3d; indice_key caching; inverse conv; AMP."""
-import os
-
+run through SparseConv3d / SubMConv3d with autograd, against torch conv3d on the densified input
+(tests.util.dense_conv_case and live); indice_key caching; inverse conv; AMP."""
 import numpy as np
 import pytest
 import torch
 
-from tests.util import random_cloud, rel_l2
+from tests.util import dense_conv_case, random_cloud, rel_l2
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 @pytest.mark.parametrize("algo_name", ["Native", "MaskImplicitGemm"])
@@ -19,7 +16,7 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden")
 def test_sparse_conv3d_equals_dense_golden(tag, k, s, p, d, algo_name, cuda_dev):
     import spconv_b200.pytorch as spconv
     from spconv_b200.core import ConvAlgo
-    g = np.load(os.path.join(GOLD, "dense_conv_case.npz"))
+    g = dense_conv_case()
     inds, feats, shape = g["inds"], g["feats"], [int(v) for v in g["shape"]]
     w, y, dy = g[f"{tag}_w"], g[f"{tag}_y"], g[f"{tag}_dy"]
     C, K = feats.shape[1], w.shape[0]
@@ -33,8 +30,8 @@ def test_sparse_conv3d_equals_dense_golden(tag, k, s, p, d, algo_name, cuda_dev)
     assert tuple(dense.shape) == y.shape
     assert np.abs(dense.detach().cpu().numpy() - y).max() < 1e-4            # test_conv.py:330
     dense.backward(torch.from_numpy(dy).to(cuda_dev))
-    # golden gradients were produced by torch dense conv3d with dy masked to the active outputs
-    # (tests/golden/make_golden.py); the sparse op defines gradients through those only
+    # the expected gradients come from torch dense conv3d with dy masked to the active outputs
+    # (tests.util.dense_conv_case); the sparse op defines gradients through those only
     ref_dw, ref_dx = g[f"{tag}_dw"], g[f"{tag}_dx"]
     assert np.abs(layer.weight.grad.cpu().numpy() - ref_dw).max() < 1e-3
     assert np.abs(x_feats.grad.cpu().numpy() - ref_dx).max() < 1e-4

@@ -2,8 +2,8 @@
 
 1. against a pure-Python transliteration of the reference CPU loops on small inputs
    (spconv/csrc/sparse/indices.py:1640-1778) -- catches C-port bugs, pins pair ORDER;
-2. against the committed golden vectors: torch dense conv3d outputs/gradients
-   (the reference's own correctness criterion, test/test_conv.py:247-357) and the
+2. against torch dense conv3d outputs/gradients on a seeded case (tests.util.dense_conv_case; the
+   reference's own correctness criterion, test/test_conv.py:247-357) and against the committed,
    independently computed facts of the reference LiDAR fixture (BASELINE.md section 2).
 """
 import json
@@ -11,6 +11,8 @@ import os
 
 import numpy as np
 import pytest
+
+from tests.util import dense_conv_case
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -150,7 +152,7 @@ def test_fixture_facts(oracle):
 def test_dense_conv_golden(oracle, tag, k, s, p, d):
     """SparseConv3d(...).dense() == nn.Conv3d on the densified input, forward and both gradients
     (test/test_conv.py:323-357, atol 1e-4 on O(1) values)."""
-    g = np.load(os.path.join(GOLD, "dense_conv_case.npz"))
+    g = dense_conv_case()
     inds, feats, shape = g["inds"], g["feats"], [int(v) for v in g["shape"]]
     w, y, dy, dw, dx = (g[f"{tag}_{n}"] for n in ("w", "y", "dy", "dw", "dx"))
     out_inds, pairs, num = oracle.get_indice_pairs(inds, 2, shape, [k] * 3, [s] * 3, [p] * 3,
@@ -161,7 +163,7 @@ def test_dense_conv_golden(oracle, tag, k, s, p, d):
     assert np.abs(got - y).max() < 1e-4
     dout = dy[out_inds[:, 0], :, out_inds[:, 1], out_inds[:, 2], out_inds[:, 3]]
     din, dwe = oracle.indice_conv_backward(feats, w, dout, pairs, num, False, False)
-    # golden gradients: torch dense conv3d backward with dy masked to the active outputs
+    # expected gradients: torch dense conv3d backward with dy masked to the active outputs
     assert np.abs(dwe - dw).max() < 1e-3
     assert np.abs(din - dx).max() < 1e-4
     # every non-active output cell of the dense conv is exactly zero

@@ -1,13 +1,21 @@
 """Point cloud -> voxel front end (SURVEY 8 f2): the CUDA generator against the REFERENCE's CPU
-generator (``Point2VoxelCPU::point_to_voxel_static``, ``spconv/csrc/sparse/pointops.py:589-695``,
-compiled into oracle/_ref) -- bit-exact: voxel order, kept points, counts, per-point ids."""
+generator (``Point2VoxelCPU::point_to_voxel_static``, ``spconv/csrc/sparse/pointops.py:589-695``)
+-- bit-exact: voxel order, kept points, counts, per-point ids.  The comparison runs against the numpy
+restatement, which must first reproduce the reference's recorded outputs (tests/golden/reference_cpu.json)."""
+import json
+import os
+
 import numpy as np
 import pytest
 import torch
 
+from tests.util import digest
+
 pytestmark = pytest.mark.gpu
 
 VS, CR = [0.4, 0.4, 0.5], [0, -40, -3, 70.4, 40, 1]          # a KITTI-like range, 8 x 200 x 176 grid
+P2V_CASES = [(20000, 3000, 5), (20000, 50000, 5), (60000, 40000, 3), (500, 100, 8)]
+GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_cpu.json")
 
 
 def _points(seed, n):
@@ -15,16 +23,17 @@ def _points(seed, n):
     return rng.uniform([-1, -41, -4, 0], [71, 41, 2, 1], size=(n, 4)).astype(np.float32)   # some out of range
 
 
-@pytest.mark.parametrize("n,max_voxels,max_points", [(20000, 3000, 5), (20000, 50000, 5), (60000, 40000, 3), (500, 100, 8)])
+@pytest.mark.parametrize("n,max_voxels,max_points", P2V_CASES)
 def test_point_to_voxel_equals_reference_cpu(n, max_voxels, max_points, oracle, cuda_dev):
     from spconv_b200.pytorch.utils import PointToVoxel, gather_features_by_pc_voxel_id
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built")
     pts = _points(n, n)
+    want = json.load(open(GOLD))["point2voxel_gpu_cases"][f"{n}/{max_voxels}x{max_points}"]
+    assert digest(pts) == want["inputs"]
     gen = PointToVoxel(VS, CR, 4, max_voxels, max_points, cuda_dev)
     assert gen.grid_size == [8, 200, 176]
     vox, ind, num, ids = gen.generate_voxel_with_id(torch.from_numpy(pts).to(cuda_dev))
-    r_vox, r_ind, r_num, r_ids = oracle.point2voxel_ref(pts, VS, CR, max_voxels, max_points)
+    r_vox, r_ind, r_num, r_ids = oracle.point2voxel(pts, VS, CR, max_voxels, max_points)
+    assert [digest(a) for a in (r_vox, r_ind, r_num, r_ids)] == want["outputs"]   # restatement == reference
     assert vox.shape[0] == r_vox.shape[0]
     assert np.array_equal(ind.cpu().numpy(), r_ind)
     assert np.array_equal(num.cpu().numpy(), r_num)
